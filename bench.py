@@ -2,12 +2,19 @@
 """Benchmark of the PV-RAFT hot path (BASELINE.json metric: RAFT iters/sec at N=8192, iters=32;
 corr-kernel HBM GB/s vs peak).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl native|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl native|reference] [--dump-outputs DIR]
 
 A "step" is one full `RSF.forward(p, num_iters=32)` (encoders + correlation build + 32 RAFT
 iterations) on a batch of synthetic N=8192 cloud pairs with seeded random-init weights.
 value = sample-iterations/s = global_batch * iters / T_forward (CUDA events, max over ranks).
 Rank 0 prints ONE JSON line.  See DESIGN.md "Measurement" for every field.
+
+--dump-outputs DIR writes what the last timed step returned as DIR/<name>.npy (float32, float64 kept), so that two builds
+can be compared output for output on identical seeded inputs:
+  inference   flows.npy [iters, B, N, 3] (RSF: the flow of every iteration) or flow.npy [B, N, 3] (RSF_refine), whole batch
+  training    loss.npy (rank 0's loss) and param.<name>.npy (every parameter after the step's Adam update)
+  reference   flows.npy [32, 1, N, 3] of the last CPU forward
+At most 64 MiB in all: a larger flow array keeps the same fixed, seeded sample of points in every sample and iteration.
 """
 import argparse
 import json
@@ -19,6 +26,7 @@ import threading
 import time
 import types
 
+import numpy as np
 import torch
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
@@ -26,6 +34,29 @@ sys.path.insert(0, ROOT)
 
 N_POINTS, TRUNC_K, ITERS, LEVELS, BASE_SCALE = 8192, 512, 32, 3, 0.25
 BATCH_PER_GPU = 8        # 8 x 32 MiB of (corr, index) state = 268 MB > the 126 MB L2: the lookup streams from HBM
+DUMP_LIMIT = 64 * 2 ** 20
+
+
+def point_sample(t, limit=DUMP_LIMIT):
+    """t [..., N, 3] of float32 cut to at most `limit` bytes: the same seeded subset of the N points (ascending) for every
+    leading index, fixed by N and the size of t alone."""
+    if t.numel() * 4 <= limit:
+        return t
+    n = t.shape[-2]
+    keep = torch.randperm(n, generator=torch.Generator().manual_seed(0))[:n * limit // (t.numel() * 4)].sort().values
+    return t.index_select(-2, keep.to(t.device))
+
+
+def dump_outputs(directory, arrays):
+    """Write every array of `arrays` (name -> tensor) as <directory>/<name>.npy: float64 stays float64, the rest is float32."""
+    host = {name: t.detach().cpu() for name, t in arrays.items()}
+    host = {name: (t if t.dtype == torch.float64 else t.float()).numpy() for name, t in host.items()}
+    total = sum(a.nbytes for a in host.values())
+    if total > DUMP_LIMIT:
+        raise ValueError(f'--dump-outputs: {total} bytes exceed the {DUMP_LIMIT} byte limit')
+    os.makedirs(directory, exist_ok=True)
+    for name, a in host.items():
+        np.save(os.path.join(directory, f'{name}.npy'), a)
 
 
 def alg_bytes_lookup(n, k, levels=LEVELS, bf16=False):
@@ -144,7 +175,7 @@ def cpu_pick_threads():
 def cpu_sample(threads, loop_iters=ITERS, n=N_POINTS):
     """One CPU sample of the bench workload at B=1: everything before the loop (encoders, graphs, correlation build) +
     `loop_iters` RAFT iterations (all 32 by default: nothing is extrapolated), timed separately.
-    Returns (t_prepare, t_loop)."""
+    Returns (t_prepare, t_loop, the flow of every iteration)."""
     from oracle import pvraft_oracle as O
     W = _cpu_weights()
     torch.set_num_threads(threads)
@@ -153,9 +184,9 @@ def cpu_sample(threads, loop_iters=ITERS, n=N_POINTS):
         t0 = time.perf_counter()
         li = O.prepare(W, pc1, pc2, TRUNC_K)
         t1 = time.perf_counter()
-        O.raft_loop(W, li, pc1, loop_iters, LEVELS, BASE_SCALE)
+        flows = O.raft_loop(W, li, pc1, loop_iters, LEVELS, BASE_SCALE)
         t2 = time.perf_counter()
-    return t1 - t0, t2 - t1
+    return t1 - t0, t2 - t1, flows
 
 
 def gpu_reference_sample(dev, batch, iters):
@@ -218,7 +249,7 @@ def gpu_reference_train_sample(dev, batch, iters):
 def run_reference(a):
     """`--impl reference`: the reference's CPU formulation (oracle port; the reference itself is pure PyTorch and is not present on
     the GPU box) timed on the host cores, same metric / unit / config.  A step is ONE full forward at B=1: the pre-loop work
-    and all 32 iterations are executed and timed (no extrapolation); steps stop early once ~200 s have been spent."""
+    and all 32 iterations are executed and timed (no extrapolation), --steps of them (each takes tens of seconds)."""
     rank = int(os.environ.get('RANK', '0'))
     if rank != 0:
         return None
@@ -227,15 +258,13 @@ def run_reference(a):
     for _ in range(warm):
         cpu_sample(threads, 1)
     t_prep = t_loop = 0.0
-    t_begin = time.perf_counter()
-    done = 0
-    for _ in range(max(1, a.steps)):
-        tp, tl = cpu_sample(threads)
+    done = a.steps
+    for _ in range(done):
+        tp, tl, flows = cpu_sample(threads)
         t_prep += tp
         t_loop += tl
-        done += 1
-        if time.perf_counter() - t_begin > 200.0:      # keep the whole arm within a few minutes
-            break
+    if a.dump_outputs:
+        dump_outputs(a.dump_outputs, {'flows': point_sample(torch.stack(flows))})
     t_prep /= done
     t_loop /= done
     value = ITERS / (t_prep + t_loop)
@@ -304,10 +333,11 @@ def run_native(a):
     pc1_h, pc2_h = pc1_h.pin_memory(), pc2_h.pin_memory()
     pc1, pc2 = pc1_h.to(dev), pc2_h.to(dev)
     out_h = torch.empty(B, N_POINTS, 3).pin_memory()
+    result = [None]      # what the latest resident step returned (--dump-outputs)
 
     def step_resident():
         with torch.no_grad():
-            return last(model([pc1, pc2], iters))
+            result[0] = model([pc1, pc2], iters)
 
     def step_e2e():
         with torch.no_grad():
@@ -338,6 +368,13 @@ def run_native(a):
     ms, launches, clocks = timed(step_resident, a.steps, sample_clocks=True)
     if clocks and set(clocks['reasons']) & {'hw_slowdown', 'hw_thermal_slowdown', 'sw_thermal_slowdown'}:
         ms, launches, clocks = timed(step_resident, a.steps, sample_clocks=True)     # re-measure once
+    if a.dump_outputs:
+        if a.refine:
+            outputs = {'flow': point_sample(D.gather_batch(result[0]))}
+        else:
+            outputs = {'flows': point_sample(torch.stack([D.gather_batch(f) for f in result[0]]))}
+        if rank == 0:
+            dump_outputs(a.dump_outputs, outputs)
     step_e2e()
     ms_e2e, _, _ = timed(step_e2e, a.steps)
     gb = B * world
@@ -411,7 +448,7 @@ def run_native(a):
         threading.Thread(target=watchdog, daemon=True).start()
     if world == 1 and not a.no_cpu:
         threads = cpu_pick_threads()
-        tp, tl = cpu_sample(threads)
+        tp, tl, _ = cpu_sample(threads)
         cpu = {'value': ITERS / (tp + tl), 'unit': 'sample-iterations/s', 'cores': threads, 'kind': 'port',
                'sample': f'one full forward at B=1, N={N_POINTS}: pre-loop work + all {ITERS} RAFT iterations, measured '
                          f'(t_prepare={tp:.2f} s, t_loop={tl:.2f} s; oracle port of the reference, torch CPU ops, '
@@ -449,6 +486,7 @@ def run_train(a):
     pc1_h, pc2_h = pc1_h.pin_memory(), pc2_h.pin_memory()
     pc1, pc2 = pc1_h.to(dev), pc2_h.to(dev)
     loss_h = torch.empty(1).pin_memory()
+    last_loss = [None]   # the latest step's loss (under graph replay: the captured step's, refreshed by every replay)
 
     def loss_fn(flows, gt, gamma=0.8):                                        # tools/loss.py:4-13 (all-ones mask)
         n = len(flows)
@@ -460,6 +498,7 @@ def run_train(a):
         loss = loss_fn(flows, x2 - x1)
         loss.backward()                                                       # DDP: the 750 KiB gradient all-reduce happens here
         opt.step()
+        last_loss[0] = loss.detach()
         return loss
 
     def step_resident():
@@ -519,6 +558,8 @@ def run_train(a):
         sampler.start()
     ms, launches = timed(step_resident, a.steps)
     clocks = sampler.stop() if sampler else None
+    if a.dump_outputs and rank == 0:
+        dump_outputs(a.dump_outputs, dict({'loss': last_loss[0]}, **{f'param.{k}': p for k, p in model.named_parameters()}))
     ms_e2e, _ = timed(step_e2e, a.steps)
     # the collective alone: one all-reduce of a gradient-sized fp32 buffer
     nparam = sum(p.numel() for p in model.parameters())
@@ -606,7 +647,11 @@ def main():
     ap.add_argument('--refine', action='store_true', help='RSF_refine instead of RSF (configs[2])')
     ap.add_argument('--no-cpu', action='store_true', help='skip the cpu_baseline leg')
     ap.add_argument('--no-gpu-ref', action='store_true', help='skip the gpu_reference leg')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help="write what the last timed step returned as DIR/<name>.npy (at most 64 MiB; see the module's docstring)")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error('--steps must be at least 1')
     if a.batch is None:
         a.batch = 2 if a.mode == 'train' else BATCH_PER_GPU
     if a.iters is None:

@@ -108,6 +108,26 @@ def trace_forward(model, pc1, pc2, iters):
     return {k: (v.detach().cpu().numpy() if torch.is_tensor(v) else v) for k, v in out.items()}
 
 
+def batch_collate():
+    """Fixture 5: the reference's collate class (datasets/generic.py:6-66) on three items of 50 points.  Loaded by file path:
+    the HuggingFace `datasets` package would shadow the reference's namespace package."""
+    import importlib.util
+    spec = importlib.util.spec_from_file_location('ref_generic', os.path.join(REF, 'datasets', 'generic.py'))
+    mod = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(mod)
+    g = torch.Generator().manual_seed(0)
+    items = [{'sequence': [torch.rand(1, 50, 3, generator=g), torch.rand(1, 50, 3, generator=g)],
+              'ground_truth': [(torch.rand(1, 50, 1, generator=g) > 0.2).float(), torch.randn(1, 50, 3, generator=g)]}
+             for _ in range(3)]
+    out = {}
+    for key in ('sequence', 'ground_truth'):
+        for ind, t in enumerate(mod.Batch(items).data[key]):
+            out[f'batch/{key}{ind}'] = t.numpy()
+            for i, it in enumerate(items):
+                out[f'item{i}/{key}{ind}'] = it[key][ind].numpy()
+    np.savez_compressed(os.path.join(HERE, 'batch_collate.npz'), **out)
+
+
 def main():
     install_scatter_shim()
     sys.path.insert(0, REF)
@@ -171,6 +191,7 @@ def main():
     idx = knn_point(16, xyz, q)
     np.savez_compressed(os.path.join(HERE, 'knn_point.npz'), xyz=xyz.numpy(), query=q.numpy(),
                         idx=np.sort(idx.numpy(), axis=-1).astype(np.int32))
+    batch_collate()
     for f in sorted(os.listdir(HERE)):
         if f.endswith('.npz'):
             print(f, os.path.getsize(os.path.join(HERE, f)) // 1024, 'KiB')

@@ -253,27 +253,14 @@ def test_weight_folds_equal_the_unfused_layers():
     assert float((got - want).abs().max() / want.abs().max()) < 1e-6
 
 
-def _items(b, n, seed=0):
-    g = torch.Generator().manual_seed(seed)
-    return [{'sequence': [torch.rand(1, n, 3, generator=g), torch.rand(1, n, 3, generator=g)],
-             'ground_truth': [(torch.rand(1, n, 1, generator=g) > 0.2).float(), torch.randn(1, n, 3, generator=g)]} for _ in range(b)]
-
-
 def test_batch_collate_matches_the_reference_class():
-    """pvraft_b200.data.Batch against datasets/generic.py:6-66 (the reference class itself when its tree is present, loaded by
-    file path because the HuggingFace `datasets` package shadows the namespace package; its documented behaviour otherwise)."""
+    """pvraft_b200.data.Batch against what the reference's class (datasets/generic.py:6-66) returned for the same three items
+    (tests/golden/batch_collate.npz, made by tests/golden/make_golden.py)."""
     from pvraft_b200.data import Batch, subsample
-    items = _items(3, 50)
+    arr, _ = load_golden('batch_collate.npz')
+    items = [{key: [arr[f'item{i}/{key}{ind}'] for ind in range(2)] for key in ('sequence', 'ground_truth')} for i in range(3)]
     mine = Batch(items)
-    ref_path = '/root/reference/datasets/generic.py'
-    if os.path.exists(ref_path):
-        import importlib.util
-        spec = importlib.util.spec_from_file_location('ref_generic', ref_path)
-        mod = importlib.util.module_from_spec(spec)
-        spec.loader.exec_module(mod)
-        ref = mod.Batch(items).data
-    else:
-        ref = {k: [torch.cat([it[k][i] for it in items], 0) for i in range(2)] for k in ('sequence', 'ground_truth')}
+    ref = {key: [arr[f'batch/{key}{ind}'] for ind in range(2)] for key in ('sequence', 'ground_truth')}
     for key in ('sequence', 'ground_truth'):
         for a, b in zip(mine[key], ref[key]):
             assert a.shape == b.shape and torch.equal(a, b)
