@@ -110,7 +110,8 @@ PVRAFT_API int pvraft_corr_reorder(const float* val_in, const int32_t* idx_in, i
  * bf16 bit patterns and candidate ids as uint16 (N <= 65536) -- 4 B instead of 8 B per candidate and iteration.  Index math
  * (coordinates, cells, kNN distances) stays fp32 and bit-exact; values are widened to fp32 exactly and accumulated in fp32, so
  * the outputs equal pvraft_corr_lookup_fwd on the bf16-rounded correlations.  K in {128,256,512,1024}.
- * pvraft_corr_state_pack_bf16 converts a reordered fp32/int32 state (round to nearest even). */
+ * pvraft_corr_state_pack_bf16 converts a reordered fp32/int32 state (round to nearest even; inf stays inf, a NaN becomes a quiet
+ * NaN of the same sign). */
 PVRAFT_API int pvraft_corr_lookup_bf16_fwd(const uint16_t* corr_val_bf16, const uint16_t* corr_idx_u16, const float* xyz2_pad,
                                 const float* coords, int B, int N, int K, int levels, float base_scale, float* vox, int vox_ld,
                                 float* knn_sel, int32_t* knn_slot, double* moments, int8_t* dbg_cube, void* stream);

@@ -364,6 +364,29 @@ def synthetic_clouds(b: int, n: int, seed: int = 1234):
     return pc1, pc2
 
 
+def randomised_affine(P: Params, seed: int, slope: Optional[float] = None) -> Params:
+    """A copy of the weights with every GroupNorm (scale, shift) and the two single-slope PReLUs redrawn.
+
+    The default init leaves every GroupNorm at (1, 0) and PReLU at 0.25, which hides sign and bias handling.  Restates
+    `tests/golden/make_golden.py:randomise_affine`, in the same parameter order: scales ~ N(0.8, 0.5) (some negative),
+    shifts ~ 0.2 N(0, 1), slopes U(0.05, 0.35) -- or `slope` for both PReLUs when given (e.g. negative, or above 1)."""
+    g = torch.Generator().manual_seed(seed)
+    out = {}
+    for name, p in P.items():
+        p = p.detach().clone()
+        if '.gn' in name or 'out_conv.1.' in name or 'knn_conv.1.' in name:
+            if name.endswith('weight'):
+                p = torch.randn(p.shape, generator=g) * 0.5 + 0.8
+            else:
+                p = torch.randn(p.shape, generator=g) * 0.2
+        if name.endswith('out_conv.2.weight') and p.numel() == 1 or name.endswith('knn_conv.2.weight'):
+            p = torch.rand(p.shape, generator=g) * 0.3 + 0.05
+            if slope is not None:
+                p = torch.full(p.shape, float(slope))
+        out[name] = p.to(P[name].dtype)
+    return out
+
+
 def synthetic_state(b: int, n: int, k: int, seed: int = 7, box: float = 3.0, jitter: float = 0.2):
     """Kernel-level state with controllable voxel density (SURVEY.md section 8d).
 

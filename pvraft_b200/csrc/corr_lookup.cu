@@ -771,7 +771,10 @@ __global__ void k_state_pack_bf16(const float* __restrict__ val, const int32_t* 
     if (i >= n) return;
     const unsigned u = __float_as_uint(__ldg(val + i));
     const unsigned r = u + 0x7FFFu + ((u >> 16) & 1u);            // round to nearest even on the dropped 16 bits
-    val_out[i] = (u & 0x7F800000u) == 0x7F800000u ? (uint16_t)(u >> 16) : (uint16_t)(r >> 16);   // inf / nan pass through
+    // inf passes through; a NaN becomes a quiet NaN with its sign kept (truncating a NaN whose payload sits in the low 16 bits
+    // would give inf)
+    const unsigned special = (u & 0x007FFFFFu) ? ((u >> 16) | 0x0040u) : (u >> 16);
+    val_out[i] = (u & 0x7F800000u) == 0x7F800000u ? (uint16_t)special : (uint16_t)(r >> 16);
     idx_out[i] = (uint16_t)__ldg(idx + i);
 }
 

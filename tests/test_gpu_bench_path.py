@@ -215,38 +215,84 @@ def test_free_running_32_iterations(dev):
     assert max(rels_own) < 2e-2, rels_own
 
 
-@pytest.mark.parametrize('n,k', [(300, 128), (1000, 256)])
-def test_ragged_point_count_model_level(dev, n, k):
+def _ragged_cases():
+    cases = []
+    for n, k in ((300, 128), (1000, 256)):
+        cases.append(pytest.param(n, k, None, id=f'{n}-{k}'))
+        cases += [pytest.param(n, k, s, id=f'{n}-{k}-randomised{s}') for s in (-0.5, 1.7)]
+    return cases
+
+
+def _model_vs_oracle(m, W, pc1, pc2, k, iters, dev):
+    """Free-running flows against the oracle, then teacher forcing through the reference-layout module seams
+    (CorrBlock.__call__, UpdateBlock.forward) on the oracle's state, graph and hidden states, then the correlation build."""
+    b, n, _ = pc1.shape
+    m.reset_graphs()
+    li = O.prepare(W, pc1, pc2, k)
+    trace = []
+    want = O.raft_loop(W, li, pc1, iters, LEVELS, SCALE, trace)
+    got = m([pc1.to(dev), pc2.to(dev)], iters)
+    worst = dict(flow=0.0, corr=0.0, net=0.0, delta=0.0)
+    for g, w in zip(got, want):
+        e = float((g.cpu() - w).abs().mean()) / float(w.abs().mean())
+        worst['flow'] = max(worst['flow'], e)
+        assert e < 2e-3
+    m.corr_block.set_state(li.state.truncated_corr.to(dev), li.state.indices.to(dev), pc2.to(dev))
+    g = product_graph(li.graph, b, n, dev)
+    net = li.net.to(dev)
+    for t in trace:
+        coords = t['coords'].to(dev).contiguous()
+        corr = m.corr_block(coords)
+        worst['corr'] = max(worst['corr'], rel_err(corr.cpu(), t['corr']))
+        assert rel_err(corr.cpu(), t['corr']) < 1e-5
+        net2, delta = m.update_block(net, li.inp.to(dev), t['corr'].to(dev), (t['coords'] - pc1).to(dev), g)
+        worst['net'] = max(worst['net'], rel_err(net2.cpu(), t['net']))
+        worst['delta'] = max(worst['delta'], rel_err(delta.cpu(), t['delta']))
+        assert rel_err(net2.cpu(), t['net']) < 1e-5
+        assert rel_err(delta.cpu(), t['delta']) < 5e-5
+        net = t['net'].to(dev)
+    # the correlation build (at a ragged N: tcgen05 GEMM on zero-padded feature maps, no library GEMM)
+    m._encode([pc1.to(dev), pc2.to(dev)])
+    assert rel_err(m.corr_block.truncated_corr.cpu(), li.state.truncated_corr) < 1e-5
+    return worst
+
+
+@pytest.mark.parametrize('n,k,slope', _ragged_cases())
+def test_ragged_point_count_model_level(dev, n, k, slope):
     """N % 128 != 0 (`--max_points` is a free flag, train.py:8-71): the CUDA-core kernels (k_corrfeat + motion stage,
     k_gru, k_flowout, k_linear) carry the loop and the padded tcgen05 GEMM builds the correlation; teacher-forced
-    module seams and free-running flows against the oracle."""
+    module seams and free-running flows against the oracle.  `slope`: every GroupNorm (scale, shift) redrawn, some scales
+    negative, and both single-slope PReLUs set to it (O.randomised_affine); None = the default init."""
     b, iters = 2, 3
     args = types.SimpleNamespace(corr_levels=LEVELS, base_scales=SCALE, truncate_k=k)
-    m, W = make_model(dev, k=k, weights=default_weights(args=args, seed=5))
+    W = default_weights(args=args, seed=5)
+    if slope is not None:
+        W = O.randomised_affine(W, seed=n, slope=slope)
+    m, W = make_model(dev, k=k, weights=W)
     pc1, pc2 = O.synthetic_clouds(b, n, seed=n)
     pc1, pc2 = pc1 * 0.3, pc2 * 0.3                  # denser cloud: non-empty voxel cells at this small N
     with torch.no_grad():
-        li = O.prepare(W, pc1, pc2, k)
-        trace = []
-        want = O.raft_loop(W, li, pc1, iters, LEVELS, SCALE, trace)
-        got = m([pc1.to(dev), pc2.to(dev)], iters)
-        for g, w in zip(got, want):
-            assert float((g.cpu() - w).abs().mean()) < 2e-3 * float(w.abs().mean())
-        # teacher-forced through the reference-layout module seams (CorrBlock.__call__, UpdateBlock.forward)
-        m.corr_block.set_state(li.state.truncated_corr.to(dev), li.state.indices.to(dev), pc2.to(dev))
-        g = product_graph(li.graph, b, n, dev)
-        net = li.net.to(dev)
-        for t in trace:
-            coords = t['coords'].to(dev).contiguous()
-            corr = m.corr_block(coords)
-            assert rel_err(corr.cpu(), t['corr']) < 1e-5
-            net2, delta = m.update_block(net, li.inp.to(dev), t['corr'].to(dev), (t['coords'] - pc1).to(dev), g)
-            assert rel_err(net2.cpu(), t['net']) < 1e-5
-            assert rel_err(delta.cpu(), t['delta']) < 5e-5
-            net = t['net'].to(dev)
-        # the correlation build of a ragged N (tcgen05 GEMM on zero-padded feature maps, no library GEMM)
-        m._encode([pc1.to(dev), pc2.to(dev)])
-        assert rel_err(m.corr_block.truncated_corr.cpu(), li.state.truncated_corr) < 1e-5
+        worst = _model_vs_oracle(m, W, pc1, pc2, k, iters, dev)
+    print(f'ragged N={n} slope={slope}: worst', {key: f'{v:.1e}' for key, v in worst.items()})
+
+
+def test_tensor_core_and_cuda_core_paths_match_oracle(dev, monkeypatch):
+    """The same N = 1024 model with randomised GroupNorm / PReLU parameters, once as shipped (every per-point layer on tcgen05)
+    and once with ops.tc_supported answering False, which routes every layer to the CUDA-core kernels that otherwise only
+    run at a ragged N.  Both against the oracle: free-running, and teacher-forced at the module seams."""
+    from pvraft_b200 import ops
+    b, n, k, iters = 2, 1024, 256, 3
+    args = types.SimpleNamespace(corr_levels=LEVELS, base_scales=SCALE, truncate_k=k)
+    W = O.randomised_affine(default_weights(args=args, seed=5), seed=n, slope=-0.5)
+    m, W = make_model(dev, k=k, weights=W)
+    pc1, pc2 = O.synthetic_clouds(b, n, seed=n)
+    pc1, pc2 = pc1 * 0.5, pc2 * 0.5
+    with torch.no_grad():
+        worst = {'tcgen05': _model_vs_oracle(m, W, pc1, pc2, k, iters, dev)}
+        monkeypatch.setattr(ops, 'tc_supported', lambda *a, **kw: False)
+        worst['cuda-core'] = _model_vs_oracle(m, W, pc1, pc2, k, iters, dev)
+    for path, w in worst.items():
+        print(f'N=1024 {path} path: worst', {key: f'{v:.1e}' for key, v in w.items()})
 
 
 def test_cuda_graph_recaptured_after_weight_update(dev):
